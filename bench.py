@@ -280,6 +280,48 @@ def parity_block(ctx, cam, cur, pools, offsets, frames):
     return out
 
 
+DUMP_BYTES = 56 << 20  # with the row indices of a sampled array (8 bytes per 132-byte row) and the .npy headers: under 64 MB
+
+
+def surfel_matrix(a):
+    """SURFEL_DTYPE records -> [n, 11] float64, columns in field order (the int32 fields are exact in float64)."""
+    return np.stack([a[f].astype(np.float64) for f in a.dtype.names], -1).reshape(len(a), len(a.dtype.names))
+
+
+def split_nonfinite(a):
+    """(a with every non-finite entry set to 0, float32 codes of the same shape: 0 finite, 1 NaN, 2 +inf, 3 -inf).
+    Surfels of a superpixel whose pixel normals are all zero carry NaN geometry, as in the reference (DESIGN.md 1.3);
+    the codes keep that information while every array written stays finite."""
+    code = np.zeros(a.shape, np.float32)
+    code[np.isnan(a)] = 1
+    code[np.isposinf(a)] = 2
+    code[np.isneginf(a)] = 3
+    return np.where(code == 0, a, 0.0), code
+
+
+def dump_outputs(outdir, ctx):
+    """What the timed batch path hands its caller after a step (dsm_batch_download): the updated local pools of all
+    frames, concatenated in frame order, and every frame's new surfels with their counts.  Written as
+    local_surfels.npy / new_surfels.npy ([n, 11] float64, columns px py pz nx ny nz size color weight update_times
+    last_update; non-finite entries written as 0 and marked in <name>_nonfinite.npy, see split_nonfinite) and
+    new_counts.npy.  Above DUMP_BYTES a fixed seeded sample of rows is kept, and <name>_rows.npy holds the indices of
+    the rows written."""
+    local, news = ctx.batch_download()
+    arrays = {"new_counts": np.array([len(n) for n in news], np.float64)}
+    for name, recs in (("local_surfels", local), ("new_surfels", np.concatenate(news))):
+        arrays[name], arrays[name + "_nonfinite"] = split_nonfinite(surfel_matrix(recs))
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(outdir, exist_ok=True)
+    for name in ("local_surfels", "new_surfels"):
+        if total > DUMP_BYTES:
+            n = len(arrays[name])
+            rows = np.sort(np.random.RandomState(0).choice(n, int(n * DUMP_BYTES / total), replace=False))
+            arrays[name], arrays[name + "_nonfinite"] = arrays[name][rows], arrays[name + "_nonfinite"][rows]
+            arrays[name + "_rows"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
 def run_extras(cam, local_rank, stream):
     """Secondary measurements reported next to the headline (not part of `value`):
     - stream: BASELINE configs[1], a sequential 1226x370 stream on the GPU-resident pool
@@ -701,6 +743,9 @@ def run_gpu_arm(args, rank, world, local_rank):
     dom_steps = max(1, int(min(dn[names.index(k)] // max(dom_launches_per_step[k], 1) for k in dom_members)))  # steps profiled on this context
     dom_ms = float(sum(dms[names.index(k)] for k in dom_members)) / dom_steps  # ms per step spent in the dominant phase
     ctx.profile_enable(0)
+    if args.dump_outputs and rank == 0:
+        # the untimed steps before the region are a multiple of the rotation (and at N>1 drain() restarts the count)
+        dump_outputs(args.dump_outputs, res_ctx[(args.steps - 1) % len(res_ctx)])
     parity = parity_block(ctx, cam, cur, pools, offsets, sorted({0, B // 3, (2 * B) // 3, B - 1})) if rank == 0 else None
     t = torch.tensor([ms_total], device=f"cuda:{local_rank}", dtype=torch.float64)
     if world > 1:
@@ -815,7 +860,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--contexts", type=int, default=None, choices=(1, 2, 3), help="resident contexts used in rotation by the timed loop (default: 2 at N=1, 3 at N>1)")
     ap.add_argument("--sub-batches", type=int, default=2, help="concurrent sub-batches of dsm_batch_run (C ABI default 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (updated local pools, new surfels, counts) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200 and at least one timed step")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

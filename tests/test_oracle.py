@@ -1,5 +1,6 @@
 """CPU tests (-m "not gpu"): the oracle against the golden vectors minted from the reference's own
-source, and the restatement against the serialised reference build when that library is present."""
+source, and the restatement against digests of what the serialised reference build returned on the
+same inputs (tests/golden/reference_serial.json)."""
 import json
 import os
 import zlib
@@ -90,48 +91,105 @@ def test_golden_stream_checksums(key, camname, flat):
         pool = np.concatenate([keep, new])
 
 
-@pytest.mark.skipif(not pyoracle.have_reference(), reason="oracle/_ref/libdsm_ref_serial.so not built")
-def test_restatement_equals_reference_serial_small():
-    """A small odd-shaped frame (W%8 == 4, H%8 == 2) with a pool: byte-identical modulo NaN payload."""
-    cam = synth.Camera(324, 242, 260.0, 260.0, 161.5, 120.5, 0.5, 30.0)
-    rs, ro = pyoracle.RefSerial(cam), pyoracle.Restatement(cam)
-    pool = np.zeros(0, SURFEL_DTYPE)
+def reference_digests(key):
+    """CRC32 digests of what the serialised reference build (oracle/_ref/libdsm_ref_serial*.so) returned on the
+    inputs of the test `key`; minted by tests/golden/make_golden.py."""
+    return json.load(open(os.path.join(GOLD, "reference_serial.json")))[key]
+
+
+def digest_stream(o, frames):
+    """fuse_initialize_map over (ref_idx, gray, depth, pose) frames, the pool carried as SurfelMap carries it; per
+    frame the CRC32 of labels, seeds, local and new surfels (NaN-canonical bytes) and the surfel counts."""
+    pool, out = np.zeros(0, SURFEL_DTYPE), []
+    for ref, g, d, pose in frames:
+        loc, new = o.fuse(ref, g, d, pose, pool)
+        out.append(dict(labels_crc=crc(o.labels()), seeds_crc=crc(canon(o.seeds())), local_crc=crc(canon(loc)),
+                        new_crc=crc(canon(new)), n_local=int(len(loc)), n_new=int(len(new))))
+        pool = np.concatenate([loc[loc["update_times"] > 0] if len(loc) else loc, new])
+    return out
+
+
+def assert_digests_equal(got, want, what):
+    assert len(got) == len(want), what
+    for t, (g, w) in enumerate(zip(got, want)):
+        bad = sorted(k for k in w if g[k] != w[k])
+        assert not bad, f"{what} frame {t}: {bad} differ from the reference"
+
+
+SMALL_CAM = synth.Camera(324, 242, 260.0, 260.0, 161.5, 120.5, 0.5, 30.0)
+RGBD_CAM = synth.Camera(324, 242, 260.0, 260.0, 161.5, 120.5, 0.3, 5.0)
+ODD_SHAPES = [(64, 48), (97, 66), (130, 83), (244, 100), (160, 124)]
+
+
+def small_frames():
+    return [(t, *synth.make_frame(SMALL_CAM, 50 + t, synth.pose_stream(t)), synth.pose_stream(t)) for t in range(3)]
+
+
+def rgbd_frames():
+    out = []
     for t in range(3):
         pose = synth.pose_stream(t)
-        g, d = synth.make_frame(cam, 50 + t, pose)
-        lr, nr = rs.fuse(t, g, d, pose, pool)
-        lo, no = ro.fuse(t, g, d, pose, pool)
-        assert (rs.labels() == ro.labels()).all()
-        assert_records_equal(ro.seeds(), rs.seeds(), "seeds")
-        assert_records_equal(lo, lr, "local")
-        assert_records_equal(no, nr, "new")
-        pool = np.concatenate([lr[lr["update_times"] > 0] if len(lr) else lr, nr])
+        g, d = synth.make_frame(RGBD_CAM, 60 + t, pose)
+        out.append((t, g, (d * np.float32(0.15)).astype(np.float32), pose))  # metres of an indoor scene
+    return out
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(pyoracle.REFDIR, "libdsm_ref_serial_rgbd.so")), reason="oracle/_ref/libdsm_ref_serial_rgbd.so not built")
+def odd_shape_camera(w, h):
+    return synth.Camera(w, h, 0.8 * w, 0.8 * w, (w - 1) / 2.0, (h - 1) / 2.0, 0.5, 30.0)
+
+
+def odd_shape_frames(cam):
+    """a carried pool and a reference-index jump (kills unstable surfels)"""
+    return [(ref, *synth.make_frame(cam, 900 + t, synth.pose_stream(t), flat=(t == 1)), synth.pose_stream(t))
+            for t, ref in enumerate([0, 1, 9])]
+
+
+def random_images():
+    """60 random 64x48 frames inside the input domain (depth 0 or >= 0.02 m): uniform noise, binary
+    salt-and-pepper, smooth ramps, with and without holes, some with many exact depth ties."""
+    yy, xx = np.mgrid[0:48, 0:64]
+    for seed in range(60):
+        rng = np.random.RandomState(seed)
+        mode = seed % 3
+        if mode == 0:
+            gray = rng.randint(0, 256, (48, 64)).astype(np.uint8)
+        elif mode == 1:
+            gray = (rng.randint(0, 2, (48, 64)) * 255).astype(np.uint8)
+        else:
+            gray = ((xx * 3 + yy * 2 + rng.randint(0, 4, (48, 64))) % 256).astype(np.uint8)
+        depth = rng.uniform(0.02, 25.0, (48, 64)).astype(np.float32)
+        if seed % 2:
+            depth[rng.rand(48, 64) < 0.4] = 0
+        if seed % 5 == 0:
+            depth = np.round(depth)  # many exact ties
+        yield gray, depth
+
+
+RANDOM_IMAGE_CAM = synth.Camera(64, 48, 60.0, 60.0, 31.5, 23.5, 0.5, 30.0)
+
+
+def digest_superpixels(o):
+    out = []
+    for gray, depth in random_images():
+        lab, seeds = o.superpixels(gray, depth)
+        out.append(dict(labels_crc=crc(lab), seeds_crc=crc(canon(seeds))))
+    return out
+
+
+def test_restatement_equals_reference_serial_small():
+    """A small odd-shaped frame (W%8 == 4, H%8 == 2) with a pool: byte-identical modulo NaN payload."""
+    assert_digests_equal(digest_stream(pyoracle.Restatement(SMALL_CAM), small_frames()), reference_digests("small"), "small")
+
+
 def test_restatement_equals_reference_serial_with_the_rgbd_constant_set():
     """The reference's second constant set (fusion_functions.h:17-21, HUBER_RANGE 0.05 ...): the restatement with
     run-time constants against the reference source compiled with those #defines, on an indoor-range stream; and the
     two sets must really differ on that data (otherwise the test would not notice a dropped constant)."""
-    cam = synth.Camera(324, 242, 260.0, 260.0, 161.5, 120.5, 0.3, 5.0)
-    rs, ro = pyoracle.RefSerialRGBD(cam), pyoracle.Restatement(cam, pyoracle.CONSTANTS_RGBD)
-    rd = pyoracle.Restatement(cam)  # drive set on the same frames
-    pool, pool_d, differs = np.zeros(0, SURFEL_DTYPE), np.zeros(0, SURFEL_DTYPE), False
-    for t in range(3):
-        pose = synth.pose_stream(t)
-        g, d = synth.make_frame(cam, 60 + t, pose)
-        d = (d * np.float32(0.15)).astype(np.float32)  # metres of an indoor scene
-        lr, nr = rs.fuse(t, g, d, pose, pool)
-        lo, no = ro.fuse(t, g, d, pose, pool)
-        assert (rs.labels() == ro.labels()).all()
-        assert_records_equal(ro.seeds(), rs.seeds(), "seeds")
-        assert_records_equal(lo, lr, "local")
-        assert_records_equal(no, nr, "new")
-        ld, nd = rd.fuse(t, g, d, pose, pool_d)
-        differs |= (rd.labels() != ro.labels()).any() or len(nd) != len(no) or canon(nd) != canon(no)
-        pool = np.concatenate([lr[lr["update_times"] > 0] if len(lr) else lr, nr])
-        pool_d = np.concatenate([ld[ld["update_times"] > 0] if len(ld) else ld, nd])
-    assert differs
+    frames = rgbd_frames()
+    got = digest_stream(pyoracle.Restatement(RGBD_CAM, pyoracle.CONSTANTS_RGBD), frames)
+    assert_digests_equal(got, reference_digests("rgbd"), "rgbd")
+    drive = digest_stream(pyoracle.Restatement(RGBD_CAM), frames)  # drive set on the same frames
+    assert any(a[k] != b[k] for a, b in zip(drive, got) for k in ("labels_crc", "new_crc", "n_new"))
 
 
 def test_every_seed_keeps_its_centre_pixel():
@@ -170,48 +228,16 @@ def test_quirks_documented_in_survey_appendix_a():
     assert lib.dsmor_create(645, 480, 1.0, 1.0, 1.0, 1.0, 30.0, 0.5) is None
 
 
-@pytest.mark.skipif(not pyoracle.have_reference(), reason="oracle/_ref/libdsm_ref_serial.so not built")
-@pytest.mark.parametrize("w,h", [(64, 48), (97, 66), (130, 83), (244, 100), (160, 124)])
+@pytest.mark.parametrize("w,h", ODD_SHAPES)
 def test_restatement_equals_reference_serial_on_odd_shapes(w, h):
     """Every supported remainder combination (W%8, H%8 in 0..4), tiny frames, a carried pool and a
     reference-index jump (kills unstable surfels): restatement == serialised reference, byte for byte."""
-    cam = synth.Camera(w, h, 0.8 * w, 0.8 * w, (w - 1) / 2.0, (h - 1) / 2.0, 0.5, 30.0)
-    rs, ro = pyoracle.RefSerial(cam), pyoracle.Restatement(cam)
-    pool = np.zeros(0, SURFEL_DTYPE)
-    for t, ref in enumerate([0, 1, 9]):
-        pose = synth.pose_stream(t)
-        g, d = synth.make_frame(cam, 900 + t, pose, flat=(t == 1))
-        lr, nr = rs.fuse(ref, g, d, pose, pool)
-        lo, no = ro.fuse(ref, g, d, pose, pool)
-        assert (rs.labels() == ro.labels()).all()
-        assert_records_equal(ro.seeds(), rs.seeds(), "seeds")
-        assert_records_equal(lo, lr, "local")
-        assert_records_equal(no, nr, "new")
-        pool = np.concatenate([lr[lr["update_times"] > 0] if len(lr) else lr, nr])
+    cam = odd_shape_camera(w, h)
+    got = digest_stream(pyoracle.Restatement(cam), odd_shape_frames(cam))
+    assert_digests_equal(got, reference_digests(f"odd_{w}x{h}"), f"{w}x{h}")
 
 
-@pytest.mark.skipif(not pyoracle.have_reference(), reason="oracle/_ref/libdsm_ref_serial.so not built")
 def test_restatement_equals_reference_serial_on_random_images():
-    """60 random 64x48 frames inside the input domain (depth 0 or >= 0.02 m): uniform noise, binary
-    salt-and-pepper, smooth ramps, with and without holes -- labels and seeds byte-identical."""
-    cam = synth.Camera(64, 48, 60.0, 60.0, 31.5, 23.5, 0.5, 30.0)
-    rs, ro = pyoracle.RefSerial(cam), pyoracle.Restatement(cam)
-    yy, xx = np.mgrid[0:48, 0:64]
-    for seed in range(60):
-        rng = np.random.RandomState(seed)
-        mode = seed % 3
-        if mode == 0:
-            gray = rng.randint(0, 256, (48, 64)).astype(np.uint8)
-        elif mode == 1:
-            gray = (rng.randint(0, 2, (48, 64)) * 255).astype(np.uint8)
-        else:
-            gray = ((xx * 3 + yy * 2 + rng.randint(0, 4, (48, 64))) % 256).astype(np.uint8)
-        depth = rng.uniform(0.02, 25.0, (48, 64)).astype(np.float32)
-        if seed % 2:
-            depth[rng.rand(48, 64) < 0.4] = 0
-        if seed % 5 == 0:
-            depth = np.round(depth)  # many exact ties
-        lab_r, seeds_r = rs.superpixels(gray, depth)
-        lab_o, seeds_o = ro.superpixels(gray, depth)
-        assert (lab_r == lab_o).all(), seed
-        assert_records_equal(seeds_o, seeds_r, f"seeds (image {seed})")
+    """The 60 random 64x48 frames of random_images(): labels and seeds byte-identical."""
+    got = digest_superpixels(pyoracle.Restatement(RANDOM_IMAGE_CAM))
+    assert_digests_equal(got, reference_digests("random_images"), "random image")
