@@ -50,15 +50,32 @@ __device__ __forceinline__ void tma_load_3d(unsigned dst, const CUtensorMap *map
                  : "memory");
 }
 
+// byte <-> bit masks of packed u8 planes
+__device__ __forceinline__ unsigned zero_bytes_to_nibble(unsigned x)
+{ // bit j of the result set iff byte j of x is zero (exact: no borrow tricks)
+    unsigned t = (x & 0x7f7f7f7fu) + 0x7f7f7f7fu;
+    t = ~(t | x | 0x7f7f7f7fu);                // 0x80 in every zero byte
+    return ((t >> 7) * 0x00204081u >> 21) & 0xfu; // bits 0, 8, 16, 24 -> bits 21..24 of the product
+}
+// 4-bit mask -> 0xff per set bit
+__device__ __forceinline__ unsigned nibble_to_bytes(unsigned n) { return (((n & 0xfu) * 0x00204081u) & 0x01010101u) * 0xffu; }
+
 // -------------------------------------------------------------------------------------------
 // K1  slic_assign (filtered) — update_pixels_kernel (:389-453) + calculate_cost (:364-387)
 //
-// A thread owns 4 consecutive pixels of one row (CTA = 64 x 2 threads = 256 x 2 pixels); the at most 2 x 2 candidate
-// seeds are shared by the four pixels.  The reference walks the image in raster order and skips a pixel whose current
-// seed is `stable` at that moment (:400); `stable` flips during the walk (:445/:450).  Here every seed carries a time
-// stamp (tstable: -1 = unstable since the start of the pass, DSM_STABLE, or the raster index at which it became
-// unstable); pixels of seeds unstable from the start commit at once, the others are deferred to the frame's relaxation
-// (SURVEY.md H1).  How the winner of a pixel is found:
+// Every pixel of the 8 x 8 block [8j+4, 8j+12) x [8k+4, 8k+12) has the same (at most) 2 x 2 candidate seeds: columns
+// {j, j+1}, rows {k, k+1} (:413-422); the pixel at column 8j+4 sees only column j (:418-420), the pixel at row 8k+4
+// only row k.  So a CTA (16 x 8 threads) covers one seed-row band, the pixel rows 8k+4 .. 8k+11 (the first band is
+// rows -4 .. 3, clipped to the image), and a run of 128 columns starting at 128a - 4; a thread owns the 8 pixels
+// 8j+4 .. 8j+11 of one row, all with the candidate columns {j, j+1}: "column 8j+4" is pixel 0 of every thread and
+// "row 8k+4" is row 0 of every band.  After pdl_enter() 17 threads build the CTA's candidate table in shared memory from
+// the band's 2 x 17 seeds (x/4, y/4, intensity, 1/mean_depth as hi + lo, mean_depth > 0); a thread then reads its
+// 2 x 2 candidates with a few LDS.  The table holds the same fp32 values the cost expressions have always used.
+// The reference walks the image in raster order and skips a pixel whose current seed is `stable` at that moment
+// (:400); `stable` flips during the walk (:445/:450).  Here every seed carries a time stamp (tstable: -1 = unstable
+// since the start of the pass, DSM_STABLE, or the raster index at which it became unstable); pixels of seeds
+// unstable from the start commit at once, the others are deferred to the frame's relaxation (SURVEY.md H1).  How the
+// winner of a pixel is found:
 //   fast path   costs in fp32 (FMA allowed).  Against the reference's value c = fl24(..fl53(..)) the fp32 value c~
 //               differs by at most 2^-20 (c~ + c) + 1e-12: squared distance and intensity term carry <= 3 roundings of
 //               2^-24 each on either side; the depth term uses 1/mean_depth as hi + lo (error 2^-48 / mean_depth,
@@ -68,7 +85,7 @@ __device__ __forceinline__ void tma_load_3d(unsigned dst, const CUtensorMap *map
 //               separated by more than that, the reference's float comparison (:427, :432, strict '<') picks the
 //               same candidate whatever the visiting order, and it is below the 1e6 start value (m1 < 9e5).
 //   exact path  everything else (ties -- common on synthetic constant images --, near ties, all costs >= 9e5):
-//               calc_cost, expression by expression as the reference.
+//               calc_cost, expression by expression as the reference, with the seeds read from global memory.
 // The first pass also writes the inverse-depth plane the later passes read instead of the depth image.
 // The last CTA of a frame to finish (ticket counter) runs the raster-order `stable` relaxation (relax_frame) for
 // that frame, so the pass needs no separate one-CTA-per-frame launch.
@@ -76,6 +93,8 @@ __device__ __forceinline__ void tma_load_3d(unsigned dst, const CUtensorMap *map
 #define A_EPS 3.814697265625e-06f // 2^-18
 #define A_ALPHA 1e-10f
 #define A_BIG 1e30f
+#define ASG_TX 16             // threads per pixel row of an assign CTA (8 rows): 128 pixel columns
+#define ASG_COLS (ASG_TX + 1) // seed columns of the CTA's candidate table
 
 __device__ __forceinline__ void relax_frame(const DsmDev &d, int b, int tid, int nthreads)
 {
@@ -115,102 +134,137 @@ __device__ __forceinline__ void relax_frame(const DsmDev &d, int b, int tid, int
     }
 }
 
-__device__ __forceinline__ float pick4(float a0, float a1, float a2, float a3, int i)
-{
-    return i == 0 ? a0 : (i == 1 ? a1 : (i == 2 ? a2 : a3));
-}
-
 // label code of a pixel: which of its (at most) 2x2 candidate seeds it is labelled with, c = 2*ix + iy over the columns
 // {xa, xa+1} and rows {ya, ya+1} defined below (the candidate set depends on the pixel position only, :413-422), or
 // DSM_CODE_NONE for a pixel the reference would have left without any label (input domain, DESIGN.md 1.3).  The u8 code
 // plane mirrors the int32 labels; the passes that only need "is this pixel a member of seed s" read it instead
 // (1 byte per pixel, and the test is a byte compare with a pattern that depends on the window position only).
 #define DSM_CODE_NONE 4
+#define DSM_CODE_NONE4 0x04040404u
+
+// seed index of candidate code c (sidx0 = seed index of candidate 0); a pixel without winner is labelled 0
+__device__ __forceinline__ int seed_of_code(unsigned c, int sidx0, int spw)
+{
+    return c == DSM_CODE_NONE ? 0 : sidx0 + (int)(c & 1u) * spw + (int)(c >> 1);
+}
+__device__ __forceinline__ int4 labels_of_codes(unsigned w, int sidx0, int spw)
+{
+    return make_int4(seed_of_code(w & 0xffu, sidx0, spw), seed_of_code((w >> 8) & 0xffu, sidx0, spw),
+                     seed_of_code((w >> 16) & 0xffu, sidx0, spw), seed_of_code(w >> 24, sidx0, spw));
+}
+// (:404-405) my_inv = (float)(1.0 / (double)depth) for depth > 0.01: 53 >= 2*24+2 bits, so the double rounding is
+// innocuous and the correctly rounded float reciprocal is the same value (-ftz=false: subnormals included)
+__device__ __forceinline__ float inv_depth(float z) { return z > F_0p01_LO ? __frcp_rn(z) : 0.0f; }
 
 template <bool FIRST>
 __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmDev d)
 {
     pdl_enter();
+    __shared__ float4 s_sd[2][ASG_COLS]; // seed rows ya, ya + 1: (x/4, or 1e18 for a missing seed; I; 1/md hi; lo)
+    __shared__ float s_syq[2][ASG_COLS]; // y/4 of the same seeds
+    __shared__ int s_md[ASG_COLS];       // bit r: the seed of row ya + r has mean_depth > 0 or is missing
     __shared__ int s_last;
     const int b = d.frame0 + blockIdx.z;
-    const int x4 = (blockIdx.x * 64 + threadIdx.x) * 4;
-    const int y = blockIdx.y * blockDim.y + threadIdx.y; // 128-thread CTAs (64 x 2): finer scheduling granularity than 256 (first pass 100.5 -> 95.2 us)
-    const int lane = threadIdx.x & 31;
-    const bool active = (x4 < d.W) && (y < d.H);
+    const int tx = threadIdx.x, ty = threadIdx.y, tid = ty * ASG_TX + tx, lane = tid & 31;
+    const int ya = (int)blockIdx.y - 1;                       // candidate seed rows {ya, ya + 1}
+    const int y = 8 * ya + 4 + ty;
+    const int xa = ASG_TX * (int)blockIdx.x - 1 + tx;         // candidate seed columns {xa, xa + 1}
+    const int x0 = 8 * xa + 4;                                // the thread's pixels x0 .. x0 + 7
+    const bool row0 = ty == 0;                                // y = 8 ya + 4 sees only seed row ya (:421-422)
+    const int spw = d.spw;
+    const int sidx0 = ya * spw + xa;                          // seed index of candidate 0
+    const size_t so = (size_t)b * d.S, fo = (size_t)b * d.px_stride;
+    const int po = y * d.Wp + x0;                             // pixel offset within the frame (H * Wp < 2^31)
+    // bit i: pixel x0 + i is inside the image.  Quad q (pixels x0 + 4q .. x0 + 4q + 3) is loaded and stored when its
+    // first pixel is: x0 + 4q is 16-byte aligned for the float planes and 4-byte aligned for the byte planes.
+    const int nx = min(d.W - x0, 8);
+    const unsigned pm = (y >= 0 && y < d.H && nx > 0) ? ((1u << nx) - 1u) & (xa < 0 ? 0xf0u : 0xffu) : 0u;
 
-    const size_t fo = (size_t)b * d.px_stride;
-    const size_t so = (size_t)b * d.S;
-    int wc[4] = {DSM_CODE_NONE, DSM_CODE_NONE, DSM_CODE_NONE, DSM_CODE_NONE}; // winner of every pixel as a candidate code
-    int oc[4] = {0, 0, 0, 0};                                                 // current label as a candidate code
-    int sidx0 = 0;                                                            // seed index of candidate 0; candidate c = sidx0 + (c & 1) * spw + (c >> 1)
-    if (active)
+    unsigned gw[2] = {0u, 0u}, ocw[2] = {0u, 0u}; // gray bytes; current labels as candidate codes (later passes)
+    float iv[8];                                  // inverse depths
+#pragma unroll
+    for (int q = 0; q < 2; q++)
     {
-        const size_t po = fo + (size_t)y * d.Wp + x4;
-        const uchar4 g4 = *reinterpret_cast<const uchar4 *>(d.gray + po);
-        float iv[4];
-        if (FIRST)
-        { // (:404-405) my_inv = (float)(1.0 / (double)depth) for depth > 0.01: 53 >= 2*24+2 bits, so the double rounding is
-          // innocuous and the correctly rounded float reciprocal is the same value (-ftz=false: subnormals included)
-            const float4 z4 = *reinterpret_cast<const float4 *>(d.depth + po);
-            iv[0] = (z4.x > F_0p01_LO) ? __frcp_rn(z4.x) : 0.0f;
-            iv[1] = (z4.y > F_0p01_LO) ? __frcp_rn(z4.y) : 0.0f;
-            iv[2] = (z4.z > F_0p01_LO) ? __frcp_rn(z4.z) : 0.0f;
-            iv[3] = (z4.w > F_0p01_LO) ? __frcp_rn(z4.w) : 0.0f;
-            *reinterpret_cast<float4 *>(d.invd + po) = make_float4(iv[0], iv[1], iv[2], iv[3]);
-        }
-        else
+        const bool ld = (pm >> (4 * q)) & 1u;
+        const int o = po + 4 * q;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (ld)
         {
-            const float4 i4 = *reinterpret_cast<const float4 *>(d.invd + po);
-            iv[0] = i4.x, iv[1] = i4.y, iv[2] = i4.z, iv[3] = i4.w;
-            const uchar4 c4 = *reinterpret_cast<const uchar4 *>(d.code + po);
-            oc[0] = c4.x, oc[1] = c4.y, oc[2] = c4.z, oc[3] = c4.w;
+            gw[q] = *reinterpret_cast<const unsigned *>(d.gray + fo + o);
+            if (FIRST)
+            {
+                v = *reinterpret_cast<const float4 *>(d.depth + fo + o);
+                v = make_float4(inv_depth(v.x), inv_depth(v.y), inv_depth(v.z), inv_depth(v.w));
+                *reinterpret_cast<float4 *>(d.invd + fo + o) = v;
+            }
+            else
+            {
+                v = *reinterpret_cast<const float4 *>(d.invd + fo + o);
+                ocw[q] = *reinterpret_cast<const unsigned *>(d.code + fo + o);
+            }
         }
-        const float gi[4] = {(float)g4.x, (float)g4.y, (float)g4.z, (float)g4.w};
-        const int bx = x4 >> 3, by = y >> 3, rx0 = x4 & 7, ry = y & 7;
-        const int xa = (rx0 == 0) ? bx - 1 : bx, xb = xa + 1;
-        const int ya = (ry < 4) ? by - 1 : by, yb = ya + 1;
-        const bool vxa = xa >= 0 && xa < d.spw, vxb = xb >= 0 && xb < d.spw;
-        const bool vya = ya >= 0 && ya < d.sph, vyb = (ry != 4) && yb >= 0 && yb < d.sph;
-        sidx0 = ya * d.spw + xa;
-        // candidate c = 2*ix + iy  -> (xa,ya) (xa,yb) (xb,ya) (xb,yb): dx outer, dy inner (:413-414)
-        // fast-path operands, shared by the thread's 4 pixels.  Coordinates are pre-scaled by 1/4 (exact), so that
-        // dist/16 (:374) is ax'^2 + ay'^2; an invalid candidate sits 1e18 away: its cost (~1e36, finite) is never the minimum
-        // and the filter arithmetic stays NaN-free.  When the pixel at x%8 == 4 sees only its own seed column (:418-420)
-        // the candidates of column xb get the same treatment for that pixel only (sxq0).
-        float sxq[4], sxq0[4], ayy[4], sI[4], shi[4], slo[4];
-        bool sv[4];
-        bool allmd = true, allmd0 = true; // every valid candidate seed has mean_depth > 0 (:378), over 4 / over column xa only
+        iv[4 * q] = v.x, iv[4 * q + 1] = v.y, iv[4 * q + 2] = v.z, iv[4 * q + 3] = v.w;
+    }
+
+    // candidate table of the band: 2 seed rows x 17 seed columns, one thread per column
+    if (tid < ASG_COLS)
+    {
+        const int j = xa - tx + tid;
+        int md = 0;
+#pragma unroll
+        for (int r = 0; r < 2; r++)
+        {
+            const int sr = ya + r;
+            const bool v = j >= 0 && j < spw && sr >= 0 && sr < d.sph;
+            // Coordinates are pre-scaled by 1/4 (exact), so that dist/16 (:374) is ax'^2 + ay'^2.  A missing candidate
+            // reads seed 0 and sits 1e18 away: its cost (~1e36, finite) is never the minimum and the filter arithmetic
+            // stays NaN-free.
+            const int li = v ? sr * spw + j : 0;
+            const float4 s4 = d.seed[so + li];
+            const float2 hl = d.seed_hl[so + li];
+            s_sd[r][tid] = make_float4(v ? s4.x * 0.25f : 1e18f, s4.z, hl.x, hl.y);
+            s_syq[r][tid] = s4.y * 0.25f;
+            md |= (s4.w > 0.f || !v) ? 1 << r : 0;
+        }
+        s_md[tid] = md;
+    }
+    __syncthreads();
+
+    unsigned wcw[2] = {DSM_CODE_NONE4, DSM_CODE_NONE4}; // winner of every pixel as a candidate code
+    if (pm)
+    {
+        // candidate c = 2*ix + iy  -> (xa,ya) (xa,yb) (xb,ya) (xb,yb): dx outer, dy inner (:413-414).  Row 0 of the band
+        // does not see row yb, pixel 0 not column xb: those candidates are pushed away like missing ones.
+        const float4 c0 = s_sd[0][tx], c1 = s_sd[1][tx], c2 = s_sd[0][tx + 1], c3 = s_sd[1][tx + 1];
+        const float sxq[4] = {c0.x, row0 ? 1e18f : c1.x, c2.x, row0 ? 1e18f : c3.x};
+        const float sI[4] = {c0.y, c1.y, c2.y, c3.y}, shi[4] = {c0.z, c1.z, c2.z, c3.z}, slo[4] = {c0.w, c1.w, c2.w, c3.w};
+        const float syq[4] = {s_syq[0][tx], s_syq[1][tx], s_syq[0][tx + 1], s_syq[1][tx + 1]};
         const float fyq = (float)y * 0.25f;
+        float ayy[4];
 #pragma unroll
         for (int c = 0; c < 4; c++)
         {
-            sv[c] = ((c >> 1) ? vxb : vxa) && ((c & 1) ? vyb : vya);
-            const int li = sv[c] ? sidx0 + (c & 1) * d.spw + (c >> 1) : 0; // invalid candidates read seed 0 and are pushed away below
-            const float4 s4 = d.seed[so + li];
-            const float2 hl = d.seed_hl[so + li];
-            sxq[c] = sv[c] ? s4.x * 0.25f : 1e18f;
-            sxq0[c] = ((c >> 1) && rx0 == 4) ? 1e18f : sxq[c];
-            const float ay = s4.y * 0.25f - fyq;
+            const float ay = syq[c] - fyq;
             ayy[c] = ay * ay;
-            sI[c] = s4.z, shi[c] = hl.x, slo[c] = hl.y;
-            const bool mdpos = s4.w > 0.f || !sv[c];
-            allmd &= mdpos;
-            if (!(c >> 1)) allmd0 &= mdpos;
         }
-        if (rx0 != 4) allmd0 = allmd;
-        unsigned uncertain = 0;
+        // every valid candidate seed has mean_depth > 0 (:378): over all 4 / over column xa only (pixel 0)
+        const int mrow = row0 ? 2 : 0;
+        const int mda = s_md[tx] | mrow, mdb = s_md[tx + 1] | mrow;
+        const bool allmd = (mda & mdb) == 3, allmd0 = mda == 3;
+        const float fxq0 = (float)x0 * 0.25f;
+        unsigned wlo = 0u, whi = 0u, uncertain = 0u;
 #pragma unroll
-        for (int i = 0; i < 4; i++)
+        for (int i = 0; i < 8; i++)
         {
-            const float fxq = (float)(x4 + i) * 0.25f;
-            const float pi = gi[i], pv = iv[i];
+            const float fxq = i == 0 ? fxq0 : fxq0 + 0.25f * (float)i; // = (float)(x0 + i) * 0.25f exactly
+            const float pi = (float)((gw[i >> 2] >> (8 * (i & 3))) & 0xffu), pv = iv[i];
             // all_has_depth (:443): every valid candidate has a depth and so has the pixel -> costs with the depth term, else without
             const float w = (pv > 0.f && (i == 0 ? allmd0 : allmd)) ? 400.f : 0.f;
             float cost[4];
 #pragma unroll
             for (int c = 0; c < 4; c++)
             {
-                const float ax = (i == 0 ? sxq0[c] : sxq[c]) - fxq;
+                const float ax = ((i == 0 && (c >> 1)) ? 1e18f : sxq[c]) - fxq;
                 const float n = fmaf(ax, ax, ayy[c]);
                 const float idf = sI[c] - pi;
                 const float cn = fmaf(idf * idf, 0.01f, n);
@@ -221,18 +275,25 @@ __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmD
             const float lo23 = fminf(cost[2], cost[3]), hi23 = fmaxf(cost[2], cost[3]);
             const float m1 = fminf(lo01, lo23);
             const float m2 = fminf(fminf(fmaxf(lo01, lo23), fminf(hi01, hi23)), A_BIG); // second smallest, kept finite
-            wc[i] = cost[0] == m1 ? 0 : (cost[1] == m1 ? 1 : (cost[2] == m1 ? 2 : 3));
+            // argmin as c = 2*ix + iy; it is used only when certain (the minimum is then unique)
+            const unsigned wc = (lo23 == m1 ? 2u : 0u) | ((cost[1] == m1 || cost[3] == m1) ? 1u : 0u);
+            if (i < 4) wlo |= wc << (8 * i);
+            else whi |= wc << (8 * (i - 4));
             const bool certain = (m2 - m1 > A_EPS * (m2 + m1) + A_ALPHA) && (m1 < 9e5f);
             if (!certain) uncertain |= 1u << i;
         }
+        uncertain &= pm;
         if (uncertain)
         { // exact path: the reference's expression, candidate order and strict '<' (first wins).  Each lane walks its OWN
           // flagged pixels, so a warp pays max-per-lane (usually one) exact evaluations, not one per pixel slot.
             SeedC sc[4];
+            bool sv[4];
 #pragma unroll
             for (int c = 0; c < 4; c++)
             {
-                const int li = sv[c] ? sidx0 + (c & 1) * d.spw + (c >> 1) : 0;
+                const int sx = xa + (c >> 1), sy = ya + (c & 1);
+                sv[c] = sx >= 0 && sx < spw && sy >= 0 && sy < d.sph && !(row0 && (c & 1));
+                const int li = sv[c] ? sy * spw + sx : 0;
                 const float4 s4 = d.seed[so + li];
                 sc[c].x = s4.x, sc[c].y = s4.y, sc[c].I = s4.z, sc[c].md = s4.w;
                 sc[c].inv = d.inv_md[so + li]; // 1.0 / (double)mean_depth, only consumed when mean_depth > 0 (:378)
@@ -242,9 +303,9 @@ __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmD
             {
                 const int i = __ffs(uncertain) - 1;
                 uncertain &= uncertain - 1;
-                const float fx = (float)(x4 + i);
-                const float my_i = pick4(gi[0], gi[1], gi[2], gi[3], i);
-                const float my_inv = pick4(iv[0], iv[1], iv[2], iv[3], i);
+                const float fx = (float)(x0 + i);
+                const float my_i = (float)d.gray[fo + po + i];
+                const float my_inv = FIRST ? inv_depth(d.depth[fo + po + i]) : d.invd[fo + po + i];
                 const double my_inv_d = (double)my_inv;
                 float min_d = 1e6f, min_nd = 1e6f;
                 int idx_d = DSM_CODE_NONE, idx_nd = DSM_CODE_NONE; // the reference's -1 (:409-411)
@@ -252,7 +313,7 @@ __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmD
 #pragma unroll
                 for (int c = 0; c < 4; c++)
                 {
-                    const bool valid = sv[c] && ((c >> 1) ? !(rx0 == 4 && i == 0) : true);
+                    const bool valid = sv[c] && !((c >> 1) && i == 0);
                     float cnd, cdd;
                     const bool has = calc_cost(sc[c], my_i, my_inv, my_inv_d, fx, fy, cnd, cdd);
                     cdd = valid ? cdd : __int_as_float(0x7f800000);
@@ -264,69 +325,70 @@ __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmD
                     min_nd = bn ? cnd : min_nd;
                     idx_nd = bn ? c : idx_nd;
                 }
-                const int wv = all_has_depth ? idx_d : idx_nd;
-                wc[0] = i == 0 ? wv : wc[0];
-                wc[1] = i == 1 ? wv : wc[1];
-                wc[2] = i == 2 ? wv : wc[2];
-                wc[3] = i == 3 ? wv : wc[3];
+                const unsigned wv = (unsigned)(all_has_depth ? idx_d : idx_nd);
+                const int sh = 8 * (i & 3);
+                if (i < 4) wlo = (wlo & ~(0xffu << sh)) | (wv << sh);
+                else whi = (whi & ~(0xffu << sh)) | (wv << sh);
             }
         }
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-            if (x4 + i >= d.W) wc[i] = DSM_CODE_NONE;
+        // pixels outside the image have no winner
+        const unsigned bm0 = nibble_to_bytes(pm), bm1 = nibble_to_bytes(pm >> 4);
+        wcw[0] = (wlo & bm0) | (DSM_CODE_NONE4 & ~bm0);
+        wcw[1] = (whi & bm1) | (DSM_CODE_NONE4 & ~bm1);
     }
-    const int spw = d.spw;
-    auto seed_of = [&](int c) { return c == DSM_CODE_NONE ? 0 : sidx0 + (c & 1) * spw + (c >> 1); }; // a pixel without winner is labelled 0
 
     if (FIRST)
     { // every label is 0 and seed 0 is unstable: everything commits (:400)
-        if (active)
-        {
-            const size_t po = fo + (size_t)y * d.Wp + x4;
-            *reinterpret_cast<int4 *>(d.labels + po) = make_int4(seed_of(wc[0]), seed_of(wc[1]), seed_of(wc[2]), seed_of(wc[3]));
-            *reinterpret_cast<uchar4 *>(d.code + po) = make_uchar4(wc[0], wc[1], wc[2], wc[3]);
-        }
+#pragma unroll
+        for (int q = 0; q < 2; q++)
+            if ((pm >> (4 * q)) & 1u)
+            {
+                *reinterpret_cast<int4 *>(d.labels + fo + po + 4 * q) = labels_of_codes(wcw[q], sidx0, spw);
+                *reinterpret_cast<unsigned *>(d.code + fo + po + 4 * q) = wcw[q];
+            }
         return;
     }
 
-    // ---- iterations 2..: commit / defer (SURVEY.md H1).  A deferred pixel whose winner IS its current label is dropped:
-    // if the raster scan evaluates it (t[label] < idx) the label does not change and the stamp t[winner] = t[label] is
-    // already below idx, so it can change nothing -- the relaxation only ever needs the pixels that would switch seeds.
-    int2 ent[4];
-    int nent = 0;
-    if (active)
+    // ---- iterations 2..: commit / defer (SURVEY.md H1).  Only a pixel whose winner differs from its label has anything
+    // to do: with winner == label an evaluated pixel keeps its label and its stamp update min(t[label], idx) is a no-op
+    // (the owner is unstable, t[label] < 0 <= idx), and a deferred one could change nothing in the relaxation either (if
+    // the raster scan evaluates it, t[label] < idx, the label does not change and the stamp t[winner] = t[label] is
+    // already below idx).  So the switching pixels are found first, from the packed codes, and the stamps are read for
+    // those few only.  (A pixel without winner keeps its label; outside the image winner and label are both NONE.)
+    unsigned sw = zero_bytes_to_nibble(~(__vcmpne4(wcw[0], ocw[0]) & __vcmpne4(wcw[0], DSM_CODE_NONE4))) |
+                  (zero_bytes_to_nibble(~(__vcmpne4(wcw[1], ocw[1]) & __vcmpne4(wcw[1], DSM_CODE_NONE4))) << 4);
+    const unsigned long long wc64 = wcw[0] | ((unsigned long long)wcw[1] << 32);
+    unsigned deferred = 0;
+    if (sw)
     {
-        bool changed = false;
         const int32_t *ts = d.tstable + so;
-        // Only a pixel whose winner differs from its label has anything to do: with winner == label an evaluated pixel
-        // keeps its label and its stamp update min(t[label], idx) is a no-op (the owner is unstable, t[label] < 0 <= idx),
-        // and a pixel of a stable owner would be deferred only to be dropped again (see above).  So the stamps are read
-        // for the few switching pixels only.
-#pragma unroll
-        for (int i = 0; i < 4; i++)
+        const unsigned long long oc64 = ocw[0] | ((unsigned long long)ocw[1] << 32);
+        unsigned long long cm = 0; // bytes of the pixels that commit
+        while (sw)
         {
-            if (x4 + i >= d.W || wc[i] == DSM_CODE_NONE || wc[i] == oc[i]) continue;
-            const int pidx = y * d.Wp + x4 + i;
-            const int win = seed_of(wc[i]);
-            if (ts[seed_of(oc[i])] < 0)
+            const int i = __ffs(sw) - 1;
+            sw &= sw - 1;
+            const int win = seed_of_code((unsigned)(wc64 >> (8 * i)) & 0xffu, sidx0, spw);
+            if (ts[seed_of_code((unsigned)(oc64 >> (8 * i)) & 0xffu, sidx0, spw)] < 0)
             { // owner unstable since the start of the pass: the reference evaluates this pixel
-                oc[i] = wc[i];
-                changed = true;
-                if (ts[win] > pidx) atomicMin(&d.tstable[so + win], pidx); // stable = false at time pidx (:445/:450)
+                cm |= 0xffull << (8 * i);
+                if (ts[win] > po + i) atomicMin(&d.tstable[so + win], po + i); // stable = false at time pidx (:445/:450)
             }
             else
+                deferred |= 1u << i;
+        }
+        const unsigned long long nc = (oc64 & ~cm) | (wc64 & cm);
+#pragma unroll
+        for (int q = 0; q < 2; q++)
+            if ((unsigned)(cm >> (32 * q)))
             {
-                ent[nent++] = make_int2(pidx, win | (wc[i] << 28));
+                const unsigned w = (unsigned)(nc >> (32 * q));
+                *reinterpret_cast<int4 *>(d.labels + fo + po + 4 * q) = labels_of_codes(w, sidx0, spw);
+                *reinterpret_cast<unsigned *>(d.code + fo + po + 4 * q) = w;
             }
-        }
-        if (changed)
-        {
-            const size_t po = fo + (size_t)y * d.Wp + x4;
-            *reinterpret_cast<int4 *>(d.labels + po) = make_int4(seed_of(oc[0]), seed_of(oc[1]), seed_of(oc[2]), seed_of(oc[3]));
-            *reinterpret_cast<uchar4 *>(d.code + po) = make_uchar4(oc[0], oc[1], oc[2], oc[3]);
-        }
     }
     // warp-aggregated append of the deferred pixels (rare: most warps have none)
+    const int nent = __popc(deferred);
     if (__any_sync(FULL, nent > 0))
     {
         int total;
@@ -334,12 +396,17 @@ __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmD
         int base = 0;
         if (lane == 31) base = atomicAdd(&d.nlist[b], total);
         base = __shfl_sync(FULL, base, 31);
-        int2 *list = d.list + fo;
-        for (int j = 0; j < nent; j++) list[base + excl + j] = ent[j];
+        int2 *list = d.list + fo + base + excl;
+        while (deferred)
+        {
+            const int i = __ffs(deferred) - 1;
+            deferred &= deferred - 1;
+            const unsigned c = (unsigned)(wc64 >> (8 * i)) & 0xffu;
+            *list++ = make_int2(po + i, seed_of_code(c, sidx0, spw) | (int)(c << 28)); // (pitched raster index, winner | code << 28)
+        }
     }
     // frame-completion ticket: the CTA that takes the last ticket of frame b sees every other CTA's labels, list
     // entries and time stamps (release: fence before the ticket; acquire: fence after it) and resolves the frame
-    const int tid = threadIdx.y * 64 + threadIdx.x;
     __syncthreads(); // the CTA's writes happen-before thread 0's fence (fences are cumulative): one fence per CTA, as in a grid barrier
     if (tid == 0)
     {
@@ -350,7 +417,7 @@ __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmD
     if (s_last)
     {
         __threadfence();
-        relax_frame(d, b, tid, 128);
+        relax_frame(d, b, tid, ASG_TX * 8);
     }
 }
 
@@ -390,12 +457,6 @@ __global__ void __launch_bounds__(128, 8) k_assign2(const __grid_constant__ DsmD
 // with the seed whose window this is.  Inside the 16 x 16 window of seed (sx, sy) the pixel at column k, row r sees that
 // seed as candidate ix = (k < 8), iy = (r < 8) (its candidate columns are {sx-1, sx} for k < 8 and {sx, sx+1} otherwise,
 // :413-422), i.e. the expected code byte is (k < 8 ? 2 : 0) | (r < 8 ? 1 : 0).  Four 32-bit words = 16 code bytes.
-__device__ __forceinline__ unsigned zero_bytes_to_nibble(unsigned x)
-{ // bit j of the result set iff byte j of x is zero (exact: no borrow tricks)
-    unsigned t = (x & 0x7f7f7f7fu) + 0x7f7f7f7fu;
-    t = ~(t | x | 0x7f7f7f7fu);                // 0x80 in every zero byte
-    return ((t >> 7) * 0x00204081u >> 21) & 0xfu; // bits 0, 8, 16, 24 -> bits 21..24 of the product
-}
 __device__ __forceinline__ unsigned member_mask16(const unsigned *codes, int r)
 {
     const unsigned lo = (r < 8) ? 0x01010101u : 0u; // iy
@@ -409,8 +470,6 @@ __device__ __forceinline__ int mask_index_sum(unsigned m)
 {
     return __popc(m & 0xaaaau) + 2 * __popc(m & 0xccccu) + 4 * __popc(m & 0xf0f0u) + 8 * __popc(m & 0xff00u);
 }
-// 4-bit mask -> 0xff per set bit
-__device__ __forceinline__ unsigned nibble_to_bytes(unsigned n) { return (((n & 0xfu) * 0x00204081u) & 0x01010101u) * 0xffu; }
 
 __global__ void __launch_bounds__(256, 6) k_gather(const __grid_constant__ DsmDev d, const __grid_constant__ DsmMaps mp)
 {
@@ -1355,8 +1414,9 @@ int dsm_tile_setup()
 }
 void dsm_launch_assign2(const DsmDev &d, int nb, bool first, cudaStream_t s)
 {
-    dim3 block(64, 2);
-    dim3 grid((d.W + 255) / 256, (d.H + 1) / 2, nb);
+    // one CTA per seed-row band (pixel rows 8k-4 .. 8k+3) and 128-column run (starting at 128a - 4)
+    dim3 block(ASG_TX, 8);
+    dim3 grid((d.W + 4 + 8 * ASG_TX - 1) / (8 * ASG_TX), (d.H + 4 + 7) / 8, nb);
     if (first)
         pdl_launch(k_assign2<true>, grid, block, 0, s, d);
     else
